@@ -60,6 +60,9 @@ def parse_args():
     p.add_argument("--no-e2e", action="store_true")
     p.add_argument("--profile", default="", help="after the timed region, run ONE extra step under torch.profiler on "
                                                  "rank 0 and write the per-kernel table to this path")
+    p.add_argument("--dump-outputs", default="", metavar="DIR",
+                   help="after the timed steps, write what the last timed step of the headline row computed as "
+                        "DIR/<name>.npy (see dump_outputs) so two builds can be compared output for output")
     return p.parse_args()
 
 
@@ -153,7 +156,35 @@ def shared_config(args, world: int, parallelism: str) -> dict:
             "grad_accum": args.accum, "optimizer": "AdamW (fp32 master + moments, grad-norm clip 1.0)", "l2": L2_NOTE}
 
 
-def _measure_ours(args, kind: str, rank: int, world: int, steps: int, with_e2e: bool, profile_path: str = "") -> dict:
+DUMP_MAX_BYTES = 64 << 20
+DUMP_SAMPLES_PER_TENSOR = 8192
+
+
+def dump_outputs(out_dir: str, loss: float, model, optimizer) -> None:
+    """Write what a training step hands back to its caller: the loss of the step (`loss.npy`, float64) and the updated
+    weights (`param.<name>.npy`, float32, one file per parameter of this rank).  A weight is read from the optimizer's
+    fp32 master copy where it keeps one of the parameter's shape (the bf16 working copy rounds small updates away),
+    otherwise from the parameter.  Tensors larger than the per-tensor budget are sampled at fixed positions that depend
+    only on the tensor's size, so equal arguments give files that can be compared element for element."""
+    import numpy as np
+    import torch
+
+    os.makedirs(out_dir, exist_ok=True)
+    np.save(os.path.join(out_dir, "loss.npy"), np.array([loss], dtype=np.float64))
+    masters = optimizer.get_working_to_master_map() or {}
+    params = list(model.unwrap().named_parameters())
+    per_tensor = min(DUMP_SAMPLES_PER_TENSOR, DUMP_MAX_BYTES // 4 // max(1, len(params)))
+    for name, p in params:
+        w = masters.get(id(p))
+        w = (w if w is not None and w.shape == p.shape else p).detach().reshape(-1)
+        if w.numel() > per_tensor:
+            idx = torch.randint(w.numel(), (per_tensor,), generator=torch.Generator().manual_seed(0)).sort().values
+            w = w[idx.to(w.device)]
+        np.save(os.path.join(out_dir, f"param.{name}.npy"), w.float().cpu().numpy())
+
+
+def _measure_ours(args, kind: str, rank: int, world: int, steps: int, with_e2e: bool, profile_path: str = "",
+                  dump_dir: str = "") -> dict:
     """Build the model under one parallel layout through the public API (Booster + HybridParallelPlugin), time
     `steps` optimizer steps, tear everything down again."""
     import gc
@@ -268,10 +299,13 @@ def _measure_ours(args, kind: str, rank: int, world: int, steps: int, with_e2e: 
     by_name = dict(launch_counter.by_name)
     clocks = sampler.stop() if rank == 0 else {}
     e2e = None
+    last_loss = loss_val
     if with_e2e:
-        ms_e, wall_e, _ = timed(steps, e2e=True)
+        ms_e, wall_e, last_loss = timed(steps, e2e=True)
         e2e = {"value": tokens_per_step * steps / (max(ms_e, wall_e) / 1e3), "unit": "tokens/s",
                "h2d_bytes_per_step": h2d_bytes, "d2h_bytes_per_step": 4, "ms_per_step": max(ms_e, wall_e) / steps}
+    if dump_dir and rank == 0:
+        dump_outputs(dump_dir, last_loss, model, optimizer)
     value = tokens_per_step * steps / (ms / 1e3)
     fused_stats = None
     if comm_backend == "fused":
@@ -313,7 +347,8 @@ def run_ours(args) -> dict:
         # the headline row runs the K steps the driver asked for; the companion row at least 3 and half of K
         steps = args.steps if i == 0 else max(3, args.steps // 2)
         rows.append(_measure_ours(args, kind, rank, world, steps, with_e2e=not args.no_e2e,
-                                  profile_path=args.profile if i == 0 else ""))
+                                  profile_path=args.profile if i == 0 else "",
+                                  dump_dir=args.dump_outputs if i == 0 else ""))
     head = rows[0]
     result = {
         "metric": METRIC, "value": head["value"], "unit": "tokens/s", "n_gpus": world, "steps": args.steps,

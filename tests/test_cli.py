@@ -7,6 +7,8 @@ import tempfile
 from colossalai_b200.cli import cli
 from colossalai_b200.cli.launcher.run import fetch_hostfile, get_launch_command, parse_device_filter
 
+ROOT = os.path.dirname(os.path.dirname(os.path.abspath(__file__)))
+
 
 def test_check_report(capsys):
     assert cli(["check", "-i"]) == 0
@@ -30,7 +32,7 @@ def test_launch_command_and_hostfile():
 def test_run_single_node(tmp_path):
     script = tmp_path / "hello.py"
     script.write_text("import os\nopen(os.environ['OUT'] + os.environ['RANK'], 'w').write(os.environ['WORLD_SIZE'])\n")
-    env = dict(os.environ, OUT=str(tmp_path / "rank"), PYTHONPATH=os.getcwd())
+    env = dict(os.environ, OUT=str(tmp_path / "rank"), PYTHONPATH=ROOT)
     r = subprocess.run([sys.executable, "-m", "colossalai_b200", "run", "--nproc_per_node", "2", "--master_port",
                         "29617", str(script)], env=env, capture_output=True, text=True, timeout=300)
     assert r.returncode == 0, r.stderr[-2000:]
